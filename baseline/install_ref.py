@@ -35,7 +35,7 @@ def verify(dst=DST):
     return True, "ok"
 
 
-def install(src="/root/reference", dst=DST, record=False):
+def install(src, dst=DST, record=False):
     if not os.path.isdir(src):
         return verify(dst)
     os.makedirs(dst, exist_ok=True)
@@ -50,6 +50,9 @@ def install(src="/root/reference", dst=DST, record=False):
 
 
 if __name__ == "__main__":
-    ok, why = install(record="--record" in sys.argv)
+    args = [a for a in sys.argv[1:] if a != "--record"]
+    if len(args) != 1:
+        sys.exit("usage: python baseline/install_ref.py <directory of the original tutorial> [--record]")
+    ok, why = install(args[0], record="--record" in sys.argv)
     print("reference install:", "OK" if ok else "FAILED", why)
     sys.exit(0 if ok else 1)

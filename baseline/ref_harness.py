@@ -34,9 +34,7 @@ ROOT = os.path.dirname(HERE)
 def load_reference():
     sys.path.insert(0, HERE)
     import install_ref
-    ok, why = install_ref.verify()
-    if not ok:
-        ok, why = install_ref.install()
+    ok, why = install_ref.verify()          # installed beforehand by install_ref.py: the benchmark writes nothing here
     if not ok:
         return None, why
     spec = importlib.util.spec_from_file_location("ref_train_dist", os.path.join(install_ref.DST, "train_dist.py"))

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark (driver contract): MNIST-ConvNet synchronous data-parallel SGD, samples/s.
 
-    python bench.py --gpus N --steps K --warmup W [--impl ours|reference]
+    python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -39,7 +39,15 @@ def parse():
     ap.add_argument("--large-batch", type=int, default=4096,
                     help="per-GPU batch of the extra large-batch (throughput, weak-scaling) measurement; 0 = skip")
     ap.add_argument("--loader-buffers", type=int, default=24, help="pinned ring depth of the native loader (e2e arm)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write what they computed (the trained parameters by name and the running "
+                         "[loss sum, #correct]) as DIR/<name>.npy, float32; inputs are seeded, so runs with the same "
+                         "arguments can be compared array for array.  Gradient sums use float atomics: after the ~500 "
+                         "steps of the default run two runs differed by up to 2.4e-3 in a weight (B200, 1000 W)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    return args
 
 
 def gpu_smi_id(torch, dev):
@@ -51,11 +59,12 @@ def gpu_smi_id(torch, dev):
         return dev.index
 
 
-def large_batch_arm(torch, b2, LB, rank, size, dev, max_over_ranks, steps=12):
-    """Device-timed samples/s of full training steps at per-GPU batch ``LB`` (weak scaling) on the batched tcgen05 engine."""
+def large_batch_arm(torch, b2, LB, rank, size, dev, max_over_ranks, steps):
+    """Device-timed samples/s of ``steps`` full training steps at per-GPU batch ``LB`` (weak scaling) on the batched
+    tcgen05 engine."""
     from dist_tuto.pth_b200.ops.convnet_batched import BatchedTrainer
     tr = BatchedTrainer(LB, lr=0.01, momentum=0.5, seed=1234, device=dev, p_drop=0.5, raw_uint8=True)
-    npool = steps + 1
+    npool = min(steps, 64) + 1                  # graphs are reused round-robin beyond 64 steps
     g = torch.Generator(device=dev).manual_seed(99 + rank)
     xs = torch.randint(0, 256, (npool, LB, 1, 28, 28), dtype=torch.uint8, device=dev, generator=g)
     ys = torch.randint(0, 10, (npool, LB), device=dev, generator=g)
@@ -82,8 +91,8 @@ def large_batch_arm(torch, b2, LB, rank, size, dev, max_over_ranks, steps=12):
         flush.fill_(1)
         graphs[0].replay()                      # pre-roll (untimed): ranks aligned by its exchange
         e0.record(st)
-        for i in range(1, npool):
-            graphs[i].replay()
+        for i in range(steps):
+            graphs[1 + i % (npool - 1)].replay()
         e1.record(st)
     st.synchronize()
     ms = max_over_ranks(e0.elapsed_time(e1), dev)
@@ -92,9 +101,18 @@ def large_batch_arm(torch, b2, LB, rank, size, dev, max_over_ranks, steps=12):
            "samples_per_s": LB * size * steps / (ms / 1e3), "dtype": "bf16 tensor-core operands (tcgen05), fp32 accumulate / master weights",
            "engine": "batched: conv2 fwd/dgrad/wgrad + fc1 on tcgen05 with TMA-fed operands, fused all-reduce+SGD kernel",
            "launches_per_step": tr.gpu_launches_per_step, "loss_finite": loss == loss,
-           "l2": "L2 flushed before the pre-roll; every timed step reads a batch not touched since"}
+           "l2": f"L2 flushed before the pre-roll; the timed steps cycle through {npool - 1} batches "
+                 f"({(npool - 1) * LB * 784 / 2**20:.0f} MB) not touched since"}
     del graphs, tr
     return out
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor as ``out_dir/<name>.npy`` in float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def ours(args):
@@ -102,7 +120,7 @@ def ours(args):
     import dist_tuto.pth_b200 as b2
     from bench_common import ClockSampler, aligned_start, max_over_ranks, result_line
     from dist_tuto.pth_b200.data import SyntheticMNIST
-    from dist_tuto.pth_b200.ops.convnet_fused import FusedTrainer
+    from dist_tuto.pth_b200.ops.convnet_fused import FusedTrainer, unpack_params
 
     K, W = args.steps, max(args.warmup, 3)
 
@@ -164,6 +182,8 @@ def ours(args):
             st.synchronize()
             b2.barrier()
             torch.cuda.synchronize()
+        if args.dump_outputs and rank == 0:        # replicas are identical: rank 0 holds what every caller receives
+            dump_outputs(args.dump_outputs, {**unpack_params(tr.params), "loss_acc": tr.loss_acc})
         ms = max_over_ranks(e0.elapsed_time(e1), dev)
         value = bsz * size * K / (ms / 1e3)
         clocks = clk.summary()
@@ -225,7 +245,7 @@ def ours(args):
         large = None
         if args.large_batch > 0:
             try:
-                large = large_batch_arm(torch, b2, args.large_batch, rank, size, dev, max_over_ranks)
+                large = large_batch_arm(torch, b2, args.large_batch, rank, size, dev, max_over_ranks, K)
             except Exception as e:      # never take the headline down
                 large = {"error": f"{type(e).__name__}: {e}"[:300]}
         if rank == 0:

@@ -37,10 +37,13 @@ def _build_locked():
     N spawned ranks all land here at once: an ``flock`` on ``csrc/build/.lock`` lets one of them build while the others
     wait and then find an up-to-date library.  ``build.build()`` is content-hashed (no-op when sources, flags and the
     link stamp match) and links to a temporary file that is ``os.replace``d into place, so nobody can import a
-    half-written library.  When nvcc is not installed (a deployment box) an existing library is used as is."""
+    half-written library.  When nvcc is not installed (a deployment box) an existing library is used as is.  An up-to-date
+    library is loaded without taking the lock, so a built tree can be used read-only."""
     import fcntl
     import shutil
     from .. import build as _b
+    if _b.up_to_date():
+        return
     have_nvcc = os.path.exists(os.path.join(_b._cuda_home(), "bin", "nvcc")) or shutil.which("nvcc") is not None
     if not have_nvcc:
         if os.path.isfile(_SO):

@@ -158,8 +158,10 @@ def train(rank: int, size: int, cfg: Optional[TrainConfig] = None):
                     copies_in_flight.popleft().synchronize()
             train_set.before_recycle = _oldest_copy_done
 
+        step_span = tracer.device_span if device.type == "cuda" else tracer.span     # CUDA events cannot time CPU work
+
         def step_fn(data, target):
-            with tracer.device_span("step", cat="step"):
+            with step_span("step", cat="step"):
                 with tracer.span("h2d"):
                     data = data.to(device, non_blocking=True)
                     target = target.to(device, non_blocking=True)
